@@ -227,6 +227,25 @@ def reduced_search_check(h, m, args):
             "witness_index": r["shards"][0]["witness_index"], "configs": r["configs"], "seconds": time.perf_counter() - t}
 
 
+def dump_outputs(path, out, shards, n_shards, rank, reduce_max):
+    """Write what the last timed step returned as float64 .npy files under `path`: the merged verdict and, per key,
+    what check_linearizable reports for it.  Timings are left out: they vary from run to run of the same build, so they
+    would hide the differences a comparison of two builds looks for."""
+    detail = np.full((4, n_shards), -1, np.int64)       # -1 = checked on another rank
+    for s, r in zip(out["mine"], shards):
+        detail[:, s] = (r["previous_ok_index"], r["cause"], r["configs"], r["probes"])
+    if reduce_max is not None:
+        detail = reduce_max(detail.ravel()).reshape(4, n_shards)
+    if rank != 0:
+        return
+    os.makedirs(path, exist_ok=True)
+    arrays = {"verdict": [out["valid"]], "shard_valid": out["shard_valid"], "shard_witness_index": out["shard_witness"],
+              "shard_previous_ok_index": detail[0], "shard_cause": detail[1], "shard_configs": detail[2],
+              "shard_probes": detail[3]}
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_reference(args, rank, world):
     if rank != 0:
         return
@@ -302,7 +321,13 @@ def main():
     ap.add_argument("--eager-reads", action="store_true",
                     help="time the product default (eager-read reduction: ~18x fewer configs, same verdict) instead of "
                          "the Knossos-exact search space the CPU reference explores")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's verdict and per-key results to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the GPU checker (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -359,6 +384,8 @@ def main():
     barrier()
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, last["shards"], h_all.n_shards, rank, reduce_max)
     # max over ranks of the times, sum over ranks of the work
     agg = torch.tensor([kern_s, wall], dtype=torch.float64, device=dev)
     tot = torch.tensor([configs, probes, algo_bytes, launches, h2d, d2h], dtype=torch.float64, device=dev)

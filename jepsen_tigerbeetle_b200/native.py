@@ -43,9 +43,18 @@ def build(force: bool = False) -> str:
     stale = (not os.path.exists(LIB_PATH)
              or any(os.path.getmtime(d) > os.path.getmtime(LIB_PATH) for d in deps))
     if force or stale:
-        cmd = ["nvcc", *NVCC_FLAGS, "-o", LIB_PATH] + [os.path.join(CSRC, f) for f in _SOURCES]
+        cmd = [_nvcc(), *NVCC_FLAGS, "-o", LIB_PATH] + [os.path.join(CSRC, f) for f in _SOURCES]
         subprocess.check_call(cmd)
     return LIB_PATH
+
+
+def _nvcc() -> str:
+    """nvcc of the CUDA toolkit PyTorch finds ($CUDA_HOME, $CUDA_PATH, nvcc on $PATH, the default install), so the
+    build works for users whose PATH lacks the toolkit's bin directory."""
+    from torch.utils.cpp_extension import CUDA_HOME
+    if CUDA_HOME is None:
+        raise NativeError("no CUDA toolkit found: set CUDA_HOME or put nvcc on PATH")
+    return os.path.join(CUDA_HOME, "bin", "nvcc")
 
 
 def lib() -> C.CDLL:

@@ -4,6 +4,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 from jepsen_tigerbeetle_b200 import abi
 from jepsen_tigerbeetle_b200.history import CModel, FlatHistory, as_c_history
@@ -11,6 +12,7 @@ from jepsen_tigerbeetle_b200.history import CModel, FlatHistory, as_c_history
 ALGO_BRUTE, ALGO_LINEAR, ALGO_WGL, ALGO_WGL_COMPACT, ALGO_LEVEL, ALGO_LAZY_BANK = 0, 1, 2, 3, 4, 5
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
+_TMP_SO = None
 
 
 def _cpu_stamp() -> str:
@@ -32,6 +34,7 @@ def _cpu_stamp() -> str:
 
 
 def build(force: bool = False) -> str:
+    global _TMP_SO
     so = os.path.join(_HERE, "libjtb_oracle.so")
     stamp_file = os.path.join(_HERE, ".build_cpu")
     srcs = [os.path.join(_HERE, f) for f in ("lin_oracle.cpp", "scan_oracle.cpp", "oracle_common.h", "Makefile")]
@@ -42,10 +45,17 @@ def build(force: bool = False) -> str:
         other_cpu = open(stamp_file).read() != stamp
     except OSError:
         other_cpu = True
-    if force or stale or other_cpu:
-        subprocess.check_call(["make", "-C", _HERE, "-B", "-s"], stdout=subprocess.DEVNULL)
-        with open(stamp_file, "w") as f:
-            f.write(stamp)
+    if not (force or stale or other_cpu):
+        return so
+    if not os.access(_HERE, os.W_OK):
+        # a read-only tree: compile once per process into a private temporary directory, leaving the tree as it is
+        if force or _TMP_SO is None:
+            _TMP_SO = os.path.join(tempfile.mkdtemp(prefix="jtb_oracle_"), "libjtb_oracle.so")
+            subprocess.check_call(["make", "-C", _HERE, "-B", "-s", "OUT=" + _TMP_SO], stdout=subprocess.DEVNULL)
+        return _TMP_SO
+    subprocess.check_call(["make", "-C", _HERE, "-B", "-s"], stdout=subprocess.DEVNULL)
+    with open(stamp_file, "w") as f:
+        f.write(stamp)
     return so
 
 

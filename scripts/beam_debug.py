@@ -1,5 +1,5 @@
-import sys, json
-sys.path.insert(0, '/root/repo')
+import sys, json, os
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from jepsen_tigerbeetle_b200 import native, synth, history as H
 sp = synth.SynthSpec('cas-register', 1000, 16, 1, p_info=0.05)
 h = synth.generate(sp); m = H.make_model(H.MODEL_CAS_REGISTER)
